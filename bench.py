@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - decoder frames/s of the wavelet-monodepth hot path on N B200s (contract: see the task brief).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--workload NAME]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--workload NAME] [--dump-outputs DIR]
 
 A "step" is one pass of the sparse wavelet decoder (SparseDepthWaveProgressiveDecoder semantics,
 thresh_ratio 0.05) over one batch of synthetic encoder features.  Headline workload (BASELINE.json
@@ -25,6 +25,7 @@ import subprocess
 import sys
 import threading
 import time
+import zlib
 
 REPO = os.path.dirname(os.path.abspath(__file__))
 if REPO not in sys.path:
@@ -48,6 +49,7 @@ SYNTH = synth.BENCH_SYNTH
 THRESH = 0.05
 METRIC, UNIT = "decoder_frames_per_sec", "frames/s"
 FP32_SIMT_PEAK_TFLOPS = 148 * 128 * 2 * 1.965e9 / 1e12      # 148 SMs x 128 FMA lanes x 2 flop x max SM clock
+DUMP_BYTES = 64 * 1000 * 1000                                # --dump-outputs: all files together
 
 
 def log(*a):
@@ -550,6 +552,37 @@ class _Stepper:
             self._finish(self.pending.pop(0))
 
 
+def output_name(key):
+    return "_".join(str(p) for p in key) if isinstance(key, tuple) else str(key)
+
+
+def dump_outputs(out, ops_result, gathered, directory, budget_bytes=DUMP_BYTES):
+    """Write one step's outputs as <directory>/<name>.npy: tensors in float32 (masks as 0 / 1), integer tensors and the
+    op counts in float64.  When the whole set exceeds `budget_bytes`, the largest tensors are cut to a fixed sample of
+    their flattened elements (positions drawn from a generator seeded by the output's name, sorted), so that two runs
+    with the same arguments write files that compare element for element."""
+    os.makedirs(directory, exist_ok=True)
+    tensors = {output_name(k): v for k, v in out.items() if torch.is_tensor(v)}
+    if gathered is not None:
+        tensors["disp_0_gathered"] = gathered
+    counts = {output_name(k): np.asarray(v, dtype=np.float64) for k, v in (ops_result or {}).items()}
+    left = budget_bytes // 8 - sum(a.size for a in counts.values()) - 64 * (len(tensors) + len(counts))
+    for name, a in counts.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+    by_size = sorted(tensors, key=lambda n: tensors[n].numel())
+    for i, name in enumerate(by_size):
+        t = tensors[name]
+        wide = t.dtype in (torch.int64, torch.int32, torch.float64)
+        cap = left // (len(by_size) - i) * (1 if wide else 2)      # `left` counts 8-byte units
+        flat = t.detach().reshape(-1)
+        if flat.numel() > cap:
+            pick = np.random.default_rng(zlib.crc32(name.encode())).choice(flat.numel(), cap, replace=False)
+            flat = flat[torch.from_numpy(np.sort(pick)).to(flat.device)]
+        left -= -(-flat.numel() // (1 if wide else 2))
+        np.save(os.path.join(directory, name + ".npy"), flat.to(torch.float64 if wide else torch.float32).cpu().numpy()
+                .reshape(t.shape if flat.numel() == t.numel() else (-1,)))
+
+
 def run_native(args, rank, world, local_rank):
     import torch.distributed as dist
     from wavelet_monodepth_b200 import _lib, graphs, ops, shard
@@ -612,6 +645,8 @@ def run_native(args, rank, world, local_rank):
     launches -= (1 if args.warmup else 0) * (launches // (args.steps + (1 if args.warmup else 0)))
     if use_graph:
         launches = graph.launches * args.steps                       # kernel nodes replayed inside the timed region
+    if args.dump_outputs and rank == 0:                              # the last timed step's outputs, before anything reuses them
+        dump_outputs(last["out"], last["ops_result"], last.get("gathered"), args.dump_outputs)
     ms_eager = time_device(eager.step, args.steps, 1, dist, world, flush=eager.flush) if use_graph else ms
     value_eager = n_global * args.steps / (ms_eager * 1e-3)
     out = last["out"]
@@ -936,7 +971,12 @@ def main():
                          "sparse levels' maps); the fastest variant is reported as e2e; 'off' skips them")
     ap.add_argument("--no-also", action="store_true")
     ap.add_argument("--no-sweep", action="store_true", help="skip the threshold sweep (configs[2] / configs[4])")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's outputs (rank 0's) as DIR/<name>.npy, at most 64 MB "
+                         "in all: larger outputs as a fixed seeded sample of their elements")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

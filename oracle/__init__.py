@@ -31,3 +31,7 @@ Pinning status (see DESIGN.md "Oracle"):
   with ``pytorch_wavelets`` proper is UNPINNED ("parity unpinned" for that
   dependency only).
 """
+
+# Intra-op threads of the process that writes and checks the golden vectors.  The CPU GEMMs split their sums by thread
+# count, so the restatement reproduces the reference's fp32 outputs bit for bit only at the count they were written with.
+GOLDEN_THREADS = 8

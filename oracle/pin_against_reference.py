@@ -29,7 +29,7 @@ import torch.nn as nn
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, REPO)
 
-from oracle import haar, kitti as okitti, nyu as onyu, sparse_ops as osp   # noqa: E402
+from oracle import GOLDEN_THREADS, haar, kitti as okitti, nyu as onyu, sparse_ops as osp   # noqa: E402
 from wavelet_monodepth_b200 import synth                                   # noqa: E402
 
 REF = "/root/reference"
@@ -339,6 +339,124 @@ def pin_state_dicts():
     print("  recorded state-dict contracts of %d reference modules" % len(rec))
 
 
+def _jsonable(v):
+    """Constructor arguments as JSON: arrays and ranges tagged so tests can rebuild the same call."""
+    if isinstance(v, np.ndarray):
+        return {"ndarray": v.tolist()}
+    if isinstance(v, range):
+        return {"range": [v.start, v.stop, v.step]}
+    if isinstance(v, (list, tuple)):
+        return [_jsonable(x) for x in v]
+    if isinstance(v, np.integer):
+        return int(v)
+    return v
+
+
+def _keys_shapes(module):
+    return [[k, list(v.shape)] for k, v in module.state_dict().items()]
+
+
+def pin_integration_seams():
+    """Record what a maintainer of the reference meets when they swap in this package's decoders (INTEGRATION.md A):
+    which class and constructor call the reference's factories make for each option set, the decoders' ``.convs`` keys,
+    the parameter groups ``pyt_utils.group_weight`` forms from them, the NYUv2 decoders' state dicts, where
+    ``load_save_utils.save_model`` writes, and the parameter names of the KITTI layer functions."""
+    import argparse as _ap
+    import contextlib
+    import inspect
+    import io
+    import tempfile
+    rec = {}
+
+    def recorders(module, names):
+        calls, orig = [], {n: getattr(module, n) for n in names}
+
+        def make(n):
+            def build(*args, **kw):
+                calls.append({"class": n, "args": _jsonable(list(args)), "kwargs": {k: _jsonable(v) for k, v in kw.items()}})
+                return orig[n](*args, **kw)
+            return build
+        for n in names:
+            setattr(module, n, make(n))
+        return calls, orig
+
+    # KITTI: networks.network_constructors.make_depth_decoder, pyt_utils.group_weight, layers.py signatures
+    layers, _ = import_reference("KITTI")
+    decs = importlib.import_module("networks.decoders")
+    ctor = importlib.import_module("networks.network_constructors")
+    pyt_utils = importlib.import_module("pyt_utils")
+    kitti_names = ("DepthDecoder", "DepthWaveProgressiveDecoder", "SparseDepthWaveProgressiveDecoder")
+    calls, orig = recorders(decs, kitti_names)
+
+    class _Encoder:
+        num_ch_enc = np.array(synth.RESNET18_CH)
+
+    factory, modules = [], {}
+    for use_wavelets, use_sparse in ((True, False), (True, True), (False, False)):
+        opts = _ap.Namespace(use_wavelets=use_wavelets, use_sparse=use_sparse, scales=range(4))
+        with contextlib.redirect_stdout(io.StringIO()):
+            m = ctor.make_depth_decoder(_Encoder(), opts)
+        call = dict(calls.pop())
+        call["opts"] = {"use_wavelets": use_wavelets, "use_sparse": use_sparse, "scales": _jsonable(opts.scales)}
+        factory.append(call)
+        groups = []
+        for _, weights in m.convs.items():
+            pyt_utils.group_weight(groups, weights, 1e-4)
+        modules[call["class"]] = {
+            "convs": [list(k) for k in m.convs.keys()],
+            "group_weight": {"decay": sum(len(g["params"]) for g in groups[0::2]),
+                             "no_decay": sum(len(g["params"]) for g in groups[1::2]), "groups": len(groups)},
+            "state_dict": _keys_shapes(m)}
+    for n, cls in orig.items():
+        setattr(decs, n, cls)
+    rec["kitti"] = {"factory": factory, "decoders": modules}
+    sigs = {}
+    for name in ("Conv3x3", "Conv1x1", "ConvBlock", "upsample", "sparse_select", "make_result", "mask2yx", "mask2idxmap",
+                 "sparse_conv1x1", "sparse_conv3x3", "sparse_upsample"):
+        a = getattr(layers, name)
+        is_class = inspect.isclass(a)
+        sigs[name] = {"class": is_class, "params": list(inspect.signature(a.__init__ if is_class else a).parameters)}
+    rec["kitti"]["layer_signatures"] = sigs
+
+    # NYUv2: model.Model and load_save_utils.save_model
+    import_reference("NYUv2")
+    decs = importlib.import_module("networks.decoders")
+    nyu_names = ("Decoder", "DecoderWave", "Decoder224", "DecoderWave224", "SparseDecoderWave")
+    for name in ("model", "load_save_utils"):
+        sys.modules.pop(name, None)
+    calls, orig = recorders(decs, nyu_names)
+    model_mod = importlib.import_module("model")
+    load_save_utils = importlib.import_module("load_save_utils")
+    cases, modules = [], {}
+    for kw in ({}, {"use_sparse": True}, {"use_224": True}, {"use_wavelets": False},
+               {"use_wavelets": False, "use_224": True}):
+        o = dict(encoder_type="densenet", normalize_input=False, pretrained_encoder=False, num_layers=18,
+                 use_wavelets=True, use_sparse=False, use_224=False, dw_waveconv=False, dw_upconv=False)
+        o.update(kw)
+        with contextlib.redirect_stdout(io.StringIO()):
+            m = model_mod.Model(_ap.Namespace(**o))
+        call = dict(calls.pop())
+        call["opts"] = o
+        cases.append(call)
+        sd = m.state_dict()
+        dec_keys = [k for k in sd if k.startswith("decoder.")]
+        assert [k[len("decoder."):] for k in dec_keys] == list(m.decoder.state_dict())
+        modules[call["class"]] = {"state_dict": _keys_shapes(m.decoder), "model_prefix": "decoder."}
+        if kw == {"use_sparse": True}:
+            with tempfile.TemporaryDirectory() as tmp, contextlib.redirect_stdout(io.StringIO()):
+                load_save_utils.save_model(m, tmp, 3)
+                written = sorted(os.path.relpath(os.path.join(d, f), tmp) for d, _, fs in os.walk(tmp) for f in fs)
+                saved = torch.load(os.path.join(tmp, written[0]))
+            assert list(saved) == list(sd)
+            rec["nyu_save_model"] = {"epoch": 3, "files": written, "content": "Model.state_dict()"}
+    for n, cls in orig.items():
+        setattr(decs, n, cls)
+    rec["nyu"] = {"model": cases, "decoders": modules}
+    with open(os.path.join(GOLDEN, "reference_seams.json"), "w") as f:
+        json.dump(rec, f, indent=0, sort_keys=False)
+    print("  recorded the integration seams (%d KITTI factory cases, %d NYUv2 model cases)" % (len(factory), len(cases)))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--skip-kat", action="store_true", help="skip the two full-size op-count runs (~10 s)")
@@ -346,6 +464,7 @@ def main():
     assert os.path.isdir(REF), "the reference checkout is only available in the build container"
     os.makedirs(GOLDEN, exist_ok=True)
     torch.set_grad_enabled(False)
+    torch.set_num_threads(GOLDEN_THREADS)
 
     def save(name, arrays, meta):
         arrays = dict(arrays)
@@ -357,6 +476,7 @@ def main():
     pin_sparse_ops(layers, save)
     pin_nyu(save)
     pin_state_dicts()
+    pin_integration_seams()
     if not args.skip_kat:
         pin_known_answers(save)
         pin_full_size()

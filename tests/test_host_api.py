@@ -110,6 +110,33 @@ def test_bench_byte_accounting_matches_the_survey_formulas():
     assert main16["operand_form"].startswith("f16x3") and main16["peak"] == 1600.0
 
 
+def test_bench_dump_outputs_fit_the_budget_and_repeat(tmp_path):
+    """--dump-outputs: every output as <name>.npy in float32 / float64, small ones whole, large ones sampled at the same
+    positions on every run, all within the byte budget."""
+    import bench
+    g = torch.Generator().manual_seed(0)
+    out = {("disp", 0): torch.rand(4, 1, 64, 256, generator=g), ("disp", 3): torch.rand(4, 1, 8, 32, generator=g),
+           ("wavelet_mask", 3): torch.rand(4, 1, 8, 32, generator=g) > 0.5, ("wavelets", 2, "LL"): torch.rand(4, 1, 32, 64),
+           "total_ops": object()}
+    ops = {"total_ops": 123456789012, "total_ops_per_sample": [1, 2, 3, 4]}
+    budget = 64 << 10
+    for run in ("a", "b"):
+        bench.dump_outputs(out, ops, None, str(tmp_path / run), budget_bytes=budget)
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == sorted(["disp_0.npy", "disp_3.npy", "wavelet_mask_3.npy", "wavelets_2_LL.npy", "total_ops.npy",
+                            "total_ops_per_sample.npy"])
+    assert sum(os.path.getsize(tmp_path / "a" / n) for n in names) <= budget
+    for n in names:
+        a, b = np.load(tmp_path / "a" / n), np.load(tmp_path / "b" / n)
+        assert a.dtype in (np.float32, np.float64) and np.array_equal(a, b)
+    assert np.array_equal(np.load(tmp_path / "a" / "disp_3.npy"), out[("disp", 3)].numpy())
+    assert np.array_equal(np.load(tmp_path / "a" / "wavelet_mask_3.npy"), out[("wavelet_mask", 3)].float().numpy())
+    assert np.load(tmp_path / "a" / "total_ops.npy") == 123456789012
+    big = np.load(tmp_path / "a" / "disp_0.npy")
+    assert big.ndim == 1 and 0 < big.size < out[("disp", 0)].numel()
+    assert np.isin(big, out[("disp", 0)].numpy().reshape(-1)).all()
+
+
 def by_sum(recs, bench):
     return sum(bench.account(name, info)[0] for name, _, info in recs)
 

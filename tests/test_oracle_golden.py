@@ -8,7 +8,7 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from oracle import haar, kitti as okitti, nyu as onyu, sparse_ops as osp
+from oracle import GOLDEN_THREADS, haar, kitti as okitti, nyu as onyu, sparse_ops as osp
 from wavelet_monodepth_b200 import synth
 from wavelet_monodepth_b200.kitti_decoders import DepthWaveProgressiveDecoder
 from wavelet_monodepth_b200.nyu_decoders import DecoderWave
@@ -17,9 +17,16 @@ from helpers import (compare_outputs, golden_names, kitti_features, load_golden,
 
 
 @pytest.fixture(autouse=True)
-def _no_grad():
-    with torch.no_grad():
-        yield
+def _golden_arithmetic():
+    """No autograd, and the thread count the fixtures were written with: on a host with more cores the default count
+    changes how the GEMMs split their sums, and the 1e-6 bar below is a same-summation-order statement."""
+    threads = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    try:
+        with torch.no_grad():
+            yield
+    finally:
+        torch.set_num_threads(threads)
 
 
 

@@ -1,116 +1,108 @@
-"""CPU, build container only: INTEGRATION.md section A executed against the UNMODIFIED reference tree.
+"""CPU: INTEGRATION.md section A, checked against what the UNMODIFIED reference does at the seams a maintainer touches.
 
-Skipped when /root/reference is absent (the GPU box).  What is checked is the seam a maintainer of the reference
-touches, not arithmetic:
-  * the three-line swap (package-level names of ``networks.decoders`` + ``sys.modules['pytorch_wavelets']``) makes the
-    reference's own factories build OUR classes: ``network_constructors.make_depth_decoder``
-    (KITTI/networks/network_constructors.py:30-40) and ``Model`` (NYUv2/model.py:47-71);
-  * ``pyt_utils.group_weight`` over ``.convs`` (KITTI/trainer.py:74-75, KITTI/pyt_utils.py:12-29) accepts every value -
-    its assert fails if a module carries a parameter that is not a Conv/Linear weight or bias;
-  * state dicts load STRICTLY in both directions (KITTI/test_simple.py:101-102) and survive the reference's own
-    save / load code paths on disk (KITTI/trainer.py:733-773 pattern, NYUv2/load_save_utils.py:10-39 called as is);
-  * without CUDA the swapped-in decoders fail loudly (no silent CPU path).
+tests/golden/reference_seams.json (written by oracle/pin_against_reference.py from the reference itself) records, for
+the reference's own factories and helpers:
+  * which decoder class, with which constructor call, ``network_constructors.make_depth_decoder``
+    (KITTI/networks/network_constructors.py:30-40) and ``Model`` (NYUv2/model.py:47-71) build for each option set -
+    after the three-line swap the same names resolve to OUR classes, so the same calls must build them;
+  * the ``.convs`` keys and the parameter groups ``pyt_utils.group_weight`` forms over them (KITTI/trainer.py:74-75,
+    KITTI/pyt_utils.py:12-29; its assert fails if a module carries a parameter that is not a Conv/Linear weight or bias);
+  * the decoders' state-dict keys and shapes, in order, so checkpoints load STRICTLY in both directions
+    (KITTI/test_simple.py:101-102) and survive the save / load code paths on disk (KITTI/trainer.py:733-773 pattern,
+    NYUv2/load_save_utils.py:10-39);
+  * the parameter names of the hot-path functions of KITTI/layers.py.
+Without CUDA the swapped-in decoders fail loudly (no silent CPU path).
 """
-import argparse
-import importlib
+import json
 import os
-import sys
 
 import numpy as np
 import pytest
 import torch
 import torch.nn as nn
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
+from wavelet_monodepth_b200 import kitti_decoders as kd
+from wavelet_monodepth_b200 import kitti_layers as kl
+from wavelet_monodepth_b200 import nyu_decoders as nd
+
+from helpers import GOLDEN
+
+SEAMS = json.load(open(os.path.join(GOLDEN, "reference_seams.json")))
+STATE_DICTS = json.load(open(os.path.join(GOLDEN, "state_dict_keys.json")))
 
 
-def _purge():
-    for name in list(sys.modules):
-        if name in ("layers", "networks", "pyt_utils", "model", "load_save_utils", "pytorch_wavelets") or \
-                name.startswith("networks."):
-            del sys.modules[name]
-    sys.path[:] = [p for p in sys.path if not p.startswith(REF)]
-    importlib.invalidate_caches()
+def _arg(v):
+    """Inverse of the pinning script's tagging: {"ndarray": [...]} -> np.array, {"range": [a, b, s]} -> range."""
+    if isinstance(v, dict) and set(v) == {"ndarray"}:
+        return np.array(v["ndarray"])
+    if isinstance(v, dict) and set(v) == {"range"}:
+        return range(*v["range"])
+    return v
 
 
-@pytest.fixture
-def kitti_tree():
-    """The reference's KITTI tree importable, `pytorch_wavelets` = our wavelets module (swap line 3)."""
-    import wavelet_monodepth_b200.wavelets as w
-    _purge()
-    sys.path.insert(0, os.path.join(REF, "KITTI"))
-    sys.modules["pytorch_wavelets"] = w
-    yield
-    _purge()
+def _build(module, call):
+    """The constructor call the reference's factory made, with the class name resolved in `module` (ours)."""
+    cls = getattr(module, call["class"])
+    return cls(*[_arg(a) for a in call["args"]], **{k: _arg(v) for k, v in call["kwargs"].items()})
 
 
-@pytest.fixture
-def nyu_tree():
-    import wavelet_monodepth_b200.wavelets as w
-    _purge()
-    sys.path.insert(0, os.path.join(REF, "NYUv2"))
-    sys.modules["pytorch_wavelets"] = w
-    yield
-    _purge()
+def _keys_shapes(module):
+    return [[k, list(v.shape)] for k, v in module.state_dict().items()]
 
 
-class _Encoder:
-    num_ch_enc = np.array([64, 64, 128, 256, 512])
+def _checkpoint_from(keys_shapes, seed):
+    """A state dict with the reference module's keys and shapes (in its order) and seeded values."""
+    g = torch.Generator().manual_seed(seed)
+    return {k: torch.randn(*shape, generator=g) for k, shape in keys_shapes}
 
 
-def _kitti_opts(**kw):
-    o = argparse.Namespace(use_wavelets=True, use_sparse=False, scales=range(4))
-    o.__dict__.update(kw)
-    return o
+def _group_counts(module):
+    """(decay, no_decay) as pyt_utils.group_weight splits a module: Conv/Linear weights, then their biases; the
+    parameters it would leave out make its assert fail, so they are checked here too."""
+    decay, no_decay = [], []
+    for m in module.modules():
+        if isinstance(m, (nn.Linear, nn.Conv2d, nn.Conv3d)):
+            decay.append(m.weight)
+            if m.bias is not None:
+                no_decay.append(m.bias)
+    assert len(list(module.parameters())) == len(decay) + len(no_decay)
+    return len(decay), len(no_decay)
 
 
-def _swap_kitti():
-    """INTEGRATION.md A, line 1: rebind the names KITTI/networks/decoders/__init__.py exports."""
-    import networks.decoders as dec
-    from wavelet_monodepth_b200 import kitti_decoders as kd
-    ref = {n: getattr(dec, n) for n in ("DepthDecoder", "DepthWaveProgressiveDecoder", "SparseDepthWaveProgressiveDecoder")}
-    for n in ref:
-        setattr(dec, n, getattr(kd, n))
-    return ref, kd
+def test_kitti_factory_builds_our_decoders_and_trainer_param_groups_accept_them():
+    assert [c["class"] for c in SEAMS["kitti"]["factory"]] == \
+        ["DepthWaveProgressiveDecoder", "SparseDepthWaveProgressiveDecoder", "DepthDecoder"]
+    for k, call in enumerate(SEAMS["kitti"]["factory"]):
+        dec = _build(kd, call)
+        want = SEAMS["kitti"]["decoders"][call["class"]]
+        decay = no_decay = groups = 0
+        for _, weights in dec.convs.items():                          # KITTI/trainer.py:74-75
+            d, nd_ = _group_counts(weights)
+            decay, no_decay, groups = decay + d, no_decay + nd_, groups + 2
+        assert {"decay": decay, "no_decay": no_decay, "groups": groups} == want["group_weight"]
+        assert decay + no_decay == len(list(dec.parameters())) > 0   # every parameter is reachable through .convs
+        assert [list(key) for key in dec.convs.keys()] == want["convs"]
+        assert _keys_shapes(dec) == want["state_dict"]
+        assert [[k_, s] for k_, s in STATE_DICTS["kitti." + call["class"]].items()] == want["state_dict"]
+        # strict loading both ways (KITTI/test_simple.py:101-102): the reference's keys and shapes, our module
+        theirs = _checkpoint_from(want["state_dict"], seed=k)
+        dec.load_state_dict(theirs, strict=True)
+        for key, v in dec.state_dict().items():
+            assert torch.equal(v, theirs[key]), key
 
 
-def test_kitti_factory_builds_our_decoders_and_trainer_param_groups_accept_them(kitti_tree, capsys):
-    ref, kd = _swap_kitti()
-    from networks.network_constructors import make_depth_decoder      # unmodified reference factory
-    from pyt_utils import group_weight                                # unmodified reference helper
-    for opts, cls in ((_kitti_opts(), kd.DepthWaveProgressiveDecoder),
-                      (_kitti_opts(use_sparse=True), kd.SparseDepthWaveProgressiveDecoder),
-                      (_kitti_opts(use_wavelets=False), kd.DepthDecoder)):
-        dec = make_depth_decoder(_Encoder(), opts)
-        assert type(dec) is cls
-        groups = []
-        for _, weights in dec.convs.items():                         # KITTI/trainer.py:74-75
-            group_weight(groups, weights, 1e-4)
-        n_grouped = sum(len(g["params"]) for g in groups)
-        assert n_grouped == len(list(dec.parameters())) > 0          # every parameter is reachable through .convs
-        refdec = ref[cls.__name__](_Encoder.num_ch_enc) if cls is kd.SparseDepthWaveProgressiveDecoder else \
-            ref[cls.__name__](_Encoder.num_ch_enc, range(4))
-        assert list(dec.state_dict().keys()) == list(refdec.state_dict().keys())
-        assert [tuple(v.shape) for v in dec.state_dict().values()] == [tuple(v.shape) for v in refdec.state_dict().values()]
-        assert list(dec.convs.keys()) == list(refdec.convs.keys())
-        # strict loading both ways (KITTI/test_simple.py:101-102)
-        dec.load_state_dict(refdec.state_dict(), strict=True)
-        refdec.load_state_dict(dec.state_dict(), strict=True)
-    capsys.readouterr()
-
-
-def test_kitti_checkpoints_round_trip_on_disk_through_the_trainers_code_path(kitti_tree, tmp_path):
-    ref, kd = _swap_kitti()
-    ours = kd.SparseDepthWaveProgressiveDecoder(_Encoder.num_ch_enc)
-    theirs = ref["SparseDepthWaveProgressiveDecoder"](_Encoder.num_ch_enc)
+def test_kitti_checkpoints_round_trip_on_disk_through_the_trainers_code_path(tmp_path):
+    ours = _build(kd, next(c for c in SEAMS["kitti"]["factory"] if c["opts"]["use_sparse"]))
+    assert type(ours) is kd.SparseDepthWaveProgressiveDecoder
+    theirs_keys = SEAMS["kitti"]["decoders"]["SparseDepthWaveProgressiveDecoder"]["state_dict"]
     # trainer.save_model (:733-751): torch.save(model.state_dict(), "<name>.pth")
     torch.save(ours.state_dict(), tmp_path / "depth.pth")
-    torch.save(theirs.state_dict(), tmp_path / "depth_ref.pth")
-    # test_simple.py:101-102: strict load of depth.pth
-    theirs.load_state_dict(torch.load(tmp_path / "depth.pth", map_location="cpu"))
+    torch.save(_checkpoint_from(theirs_keys, seed=5), tmp_path / "depth_ref.pth")
+    # what a reference module loading depth.pth strictly requires: exactly its keys, in its order, with its shapes
+    mine = torch.load(tmp_path / "depth.pth", map_location="cpu")
+    assert [[k, list(v.shape)] for k, v in mine.items()] == theirs_keys
     for k, v in ours.state_dict().items():
-        assert torch.equal(theirs.state_dict()[k], v), k
+        assert torch.equal(mine[k], v), k
     # trainer.load_model (:753-773): filter by key, update, load
     model_dict = ours.state_dict()
     pretrained = {k: v for k, v in torch.load(tmp_path / "depth_ref.pth").items() if k in model_dict}
@@ -123,73 +115,73 @@ def test_kitti_checkpoints_round_trip_on_disk_through_the_trainers_code_path(kit
     ours.load_state_dict(torch.load(tmp_path / "depth_ref.pth"), strict=False)
 
 
-def test_swapped_kitti_decoder_fails_loudly_without_cuda(kitti_tree):
-    if torch.cuda.is_available():
-        pytest.skip("CUDA present")
-    _, kd = _swap_kitti()
+def test_swapped_kitti_decoder_fails_loudly_without_cuda():
+    """Host tensors are refused whether or not a device is present: there is no CPU path to fall back to."""
     from wavelet_monodepth_b200._lib import WmdError
-    dec = kd.SparseDepthWaveProgressiveDecoder(_Encoder.num_ch_enc)
-    feats = [torch.rand(1, c, 6 << (4 - k), 20 << (4 - k)) for k, c in enumerate(_Encoder.num_ch_enc)]
+    call = next(c for c in SEAMS["kitti"]["factory"] if c["opts"]["use_sparse"])
+    dec = _build(kd, call)
+    num_ch_enc = _arg(call["args"][0])
+    feats = [torch.rand(1, c, 6 << (4 - k), 20 << (4 - k)) for k, c in enumerate(num_ch_enc)]
     with pytest.raises(WmdError):
         dec(feats, 0.05)
 
 
-def _nyu_opts(**kw):
-    o = argparse.Namespace(encoder_type="densenet", normalize_input=False, pretrained_encoder=False, num_layers=18,
-                           use_wavelets=True, use_sparse=False, use_224=False, dw_waveconv=False, dw_upconv=False)
-    o.__dict__.update(kw)
-    return o
+class _Model(nn.Module):
+    """Stand-in for NYUv2/model.py's Model: the decoder under `decoder.`, beside an encoder."""
+
+    def __init__(self, decoder):
+        super().__init__()
+        self.encoder = nn.Conv2d(3, 4, 3)
+        self.decoder = decoder
 
 
-def test_nyu_model_builds_our_decoders_and_load_save_utils_round_trip(nyu_tree, tmp_path, capsys):
-    import networks.decoders as dec
-    from wavelet_monodepth_b200 import nyu_decoders as nd
-    ref = {n: getattr(dec, n) for n in ("Decoder", "DecoderWave", "Decoder224", "DecoderWave224", "SparseDecoderWave")}
-    for n in ref:                                                    # INTEGRATION.md A, line 2
-        setattr(dec, n, getattr(nd, n))
-    from model import Model                                          # unmodified NYUv2/model.py
-    import load_save_utils                                           # unmodified NYUv2/load_save_utils.py
-    cases = ((_nyu_opts(), nd.DecoderWave), (_nyu_opts(use_sparse=True), nd.SparseDecoderWave),
-             (_nyu_opts(use_224=True), nd.DecoderWave224), (_nyu_opts(use_wavelets=False), nd.Decoder),
-             (_nyu_opts(use_wavelets=False, use_224=True), nd.Decoder224))
-    enc_ch = None
-    for opts, cls in cases:
-        m = Model(opts)
-        assert type(m.decoder) is cls
-        enc_ch = list(m.encoder.num_ch_enc)
-        theirs = ref[cls.__name__](enc_features=enc_ch, decoder_width=0.5)
-        assert list(m.decoder.state_dict().keys()) == list(theirs.state_dict().keys()), cls.__name__
-        assert [tuple(v.shape) for v in m.decoder.state_dict().values()] == \
-               [tuple(v.shape) for v in theirs.state_dict().values()]
-        m.decoder.load_state_dict(theirs.state_dict(), strict=True)
-        theirs.load_state_dict(m.decoder.state_dict(), strict=True)
-    # the reference's own save_model / load_model on a model that carries our decoder, then into a pure-reference twin
-    m = Model(_nyu_opts(use_sparse=True))
-    load_save_utils.save_model(m, str(tmp_path), 3)                  # writes models/weights_3/model.pth
-    folder = os.path.join(str(tmp_path), "models", "weights_3")
-    import model as model_module
-    for n in ref:                                                    # back to the reference's classes (model.py bound
-        setattr(model_module, n, ref[n])                             # the names at import time)
-    twin = Model(_nyu_opts(use_sparse=True))
-    assert type(twin.decoder) is ref["SparseDecoderWave"]
-    load_save_utils.load_model(twin, folder)
-    for k, v in m.state_dict().items():
-        assert torch.equal(twin.state_dict()[k], v), k
-    load_save_utils.save_model(twin, str(tmp_path), 4)
-    load_save_utils.load_model(m, os.path.join(str(tmp_path), "models", "weights_4"))
-    capsys.readouterr()
+def test_nyu_model_builds_our_decoders_and_load_save_utils_round_trip(tmp_path):
+    cases = SEAMS["nyu"]["model"]
+    assert [c["class"] for c in cases] == ["DecoderWave", "SparseDecoderWave", "DecoderWave224", "Decoder", "Decoder224"]
+    for k, call in enumerate(cases):
+        dec = _build(nd, call)                                       # INTEGRATION.md A, line 2
+        want = SEAMS["nyu"]["decoders"][call["class"]]["state_dict"]
+        assert _keys_shapes(dec) == want, call["class"]
+        theirs = _checkpoint_from(want, seed=k)
+        dec.load_state_dict(theirs, strict=True)
+        for key, v in dec.state_dict().items():
+            assert torch.equal(v, theirs[key]), key
+        if "nyu." + call["class"] in STATE_DICTS:
+            assert [[k_, s] for k_, s in STATE_DICTS["nyu." + call["class"]].items()] == want
+    # load_save_utils.save_model writes Model.state_dict() to <log>/models/weights_<epoch>/model.pth and load_model
+    # filters a checkpoint by the model's keys, updates and loads it: a model carrying our decoder, then a reference twin
+    save = SEAMS["nyu_save_model"]
+    assert save["files"] == ["models/weights_%d/model.pth" % save["epoch"]]
+    sparse = next(c for c in cases if c["class"] == "SparseDecoderWave")
+    m = _Model(_build(nd, sparse))
+    path = tmp_path / save["files"][0]
+    path.parent.mkdir(parents=True)
+    torch.save(m.state_dict(), path)
+    prefix = SEAMS["nyu"]["decoders"]["SparseDecoderWave"]["model_prefix"]
+    saved = torch.load(path)
+    theirs_keys = SEAMS["nyu"]["decoders"]["SparseDecoderWave"]["state_dict"]
+    assert [[k[len(prefix):], list(v.shape)] for k, v in saved.items() if k.startswith(prefix)] == theirs_keys
+    twin = {prefix + k: v for k, v in _checkpoint_from(theirs_keys, seed=9).items()}
+    torch.save(twin, tmp_path / "twin.pth")
+    model_dict = m.state_dict()
+    pretrained = {k: v for k, v in torch.load(tmp_path / "twin.pth").items() if k in model_dict}
+    assert set(pretrained) == {k for k in model_dict if k.startswith(prefix)}
+    model_dict.update(pretrained)
+    m.load_state_dict(model_dict)
+    for k, v in twin.items():
+        assert torch.equal(m.state_dict()[k], v), k
 
 
-def test_functional_api_names_match_the_reference_layers(kitti_tree):
+def test_functional_api_names_match_the_reference_layers():
     """Every public name of the hot path in KITTI/layers.py exists with the same parameter names here."""
     import inspect
-    import layers as ref_layers
-    from wavelet_monodepth_b200 import kitti_layers as kl
-    for name in ("Conv3x3", "Conv1x1", "ConvBlock", "upsample", "sparse_select", "make_result", "mask2yx", "mask2idxmap",
-                 "sparse_conv1x1", "sparse_conv3x3", "sparse_upsample"):
-        a, b = getattr(ref_layers, name), getattr(kl, name)
-        if inspect.isclass(a):
-            assert issubclass(b, nn.Module)
-            a, b = a.__init__, b.__init__
-        pa, pb = list(inspect.signature(a).parameters), list(inspect.signature(b).parameters)
+    sigs = SEAMS["kitti"]["layer_signatures"]
+    assert sorted(sigs) == sorted(("Conv3x3", "Conv1x1", "ConvBlock", "upsample", "sparse_select", "make_result", "mask2yx",
+                                   "mask2idxmap", "sparse_conv1x1", "sparse_conv3x3", "sparse_upsample"))
+    for name, want in sigs.items():
+        b = getattr(kl, name)
+        if want["class"]:
+            assert inspect.isclass(b) and issubclass(b, nn.Module), name
+            b = b.__init__
+        pa, pb = want["params"], list(inspect.signature(b).parameters)
         assert pa == pb[:len(pa)], (name, pa, pb)
