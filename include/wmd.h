@@ -192,14 +192,15 @@ typedef struct wmd_conv_desc {
   float* amax_out;          /* device scalar, or NULL: atomically raised to max |y| of the rows written (zero it before the
                                first producer; both precisions) */
   int32_t rows0;            /* rows allocated in x0, 0 = unknown.  Only used by the tensor-core engine's 1x1 form (taps == 1,
-                               map0 == NULL: output row m reads x0 row m): with rows0 > 0 it loads whole 256-row tiles by TMA
-                               (reads past rows0 are zero-filled) instead of gathering row by row */
+                               map0 == NULL: output row m reads x0 row m) without a gate: with rows0 > 0 it loads source 0 in
+                               whole 256-row tiles by TMA (reads past rows0 are zero-filled) instead of gathering row by row */
 } wmd_conv_desc;
 
 int wmd_conv_rows_f32(const wmd_conv_desc* d, wmd_stream_t stream);
 
 /* Tensor-core engine for the same contract: tcgen05.mma.kind::tf32 with a 3xTF32 split (hi*hi + lo*hi + hi*lo,
- * fp32 accumulation in TMEM), so results stay fp32-faithful (<= ~1e-6 relative vs the SIMT kernel).  d->w must
+ * fp32 accumulation in TMEM), so results stay fp32-faithful: max|y - ref| / max|ref| <= 8e-6 against an fp64 reference
+ * at any K (4e-6 in the f16x3 form; the SIMT kernel: 1.2e-6), measured on B200 by tests/test_gpu_conv_reference.py.  d->w must
  * point to weights packed by wmd_pack_conv_weight_tc_f32 for the same (cout, c0, c1, taps); d->ldw is ignored.
  *   wmd_conv_tc_tile_n(cout)                 N-tile of the kernel for this cout (128 / 64 / 32; the CTA tile is 256 rows x N)
  *   wmd_conv_tc_weight_floats(...)           size of the packed weight buffer, in floats

@@ -395,7 +395,9 @@ __global__ void __launch_bounds__(TC_THREADS, 1) conv_rows_tc_kernel(const wmd_c
   const long long tiles = static_cast<long long>((rows + TC_BM - 1) / TC_BM) * n_tiles;
   const int Hs = d.H >> d.shift0, Ws = d.W >> d.shift0;
   const bool aligned_rows = (d.taps == 1 && d.map0 == nullptr);
-  const bool tiled_rows = aligned_rows && d.rows0 > 0;         // tm0 then has a 256-row box (launch_tc)
+  // tm0 then has a 256-row box (launch_tc).  A box load cannot zero gated-off rows, so a gate takes the per-row gathers;
+  // source-1 chunks always go through the tap table
+  const bool tiled_rows = aligned_rows && d.rows0 > 0 && d.gate == nullptr;
   // instruction descriptor: D=f32, A=B=tf32, both K-major, N = BN, M = 128
   // (F16: A = B = f16, format code 0, K = 16 per instruction)
   constexpr uint32_t kFmt = F16 ? 0u : 2u;
@@ -643,7 +645,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) conv_rows_tc_kernel(const wmd_c
     constexpr int kMaxLoadsPerWarp = (TC_BM / 4 + TC_GATHER_WARPS - 1) / TC_GATHER_WARPS;
     auto gather_chunk = [&](int c, uint32_t round) {
       const uint32_t st = round % TC_A_STAGES;
-      if (tiled_rows) {
+      if (tiled_rows && c < nch0) {
         // 1x1 stages read tile rows m0 .. m0+255 of x0 as they are: ONE tiled TMA load (box = 256 rows x 32 channels, tm0 is
         // encoded with that box by the host) instead of 64 four-row gathers - 690 vs 974 clk per chunk measured
         // (scripts/bench_cu/tma_tile_rate.cu) and no issue pressure.  Rows past the tensor / channels past C read zeros.
@@ -1372,8 +1374,8 @@ static int launch_tc(const wmd_conv_desc& d, int splits, float* partial, cudaStr
   {
     const long long px = static_cast<long long>(d.N) * d.H * d.W;
     const long long rows0 = static_cast<long long>(d.N) * (d.H >> d.shift0) * (d.W >> d.shift0);
-    // 1x1 stage over its own rows (taps == 1, no index map): the kernel loads whole 256-row tiles
-    const bool tiled = (d.taps == 1 && d.map0 == nullptr && d.rows0 > 0);
+    // 1x1 stage over its own rows (taps == 1, no index map, no gate): the kernel loads whole 256-row tiles of source 0
+    const bool tiled = (d.taps == 1 && d.map0 == nullptr && d.rows0 > 0 && d.gate == nullptr);
     int rc = make_rows_map(&tm0, d.x0, d.c0, tiled ? d.rows0 : rows0, d.ld0, tiled ? TC_BM : 1);
     if (rc != WMD_OK) return rc;
     if (d.c1 > 0) {
